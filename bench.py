@@ -8,8 +8,11 @@ resident in HBM; `e2e` times the same call through the C ABI with HOST buffers (
 device, apply, device y -> host) every step. `--impl reference` times the reference's own
 algorithm (dense non-tensor basis, the CPU oracle port) on the host cores.
 
-Launch:  python bench.py [--gpus N --steps K --warmup W]   or, for N > 1,
+Launch:  python bench.py [--gpus N --steps K --warmup W] [--dump-outputs DIR]   or, for N > 1,
          python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes the y of the last timed step as DIR/y.npy (DIR/y_rank<r>.npy per rank for N > 1), float64. x, the mesh
+and the coefficients are fixed by the arguments, so two builds can be compared output for output, and the two arms with each other.
 """
 from __future__ import annotations
 
@@ -25,9 +28,13 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the tree may be read-only: no bytecode caches from this process or the experiments' child processes
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 METRIC = "curl-curl+mass operator apply throughput"
 UNIT = "MDoF/s"
+DUMP_BYTES = 64 << 20  # --dump-outputs: at most this much over all ranks
 
 
 def parse():
@@ -46,7 +53,23 @@ def parse():
     ap.add_argument("--cpu-sample-elems", type=int, default=0, help="elements in the CPU baseline sample (0 = auto)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-experiments", action="store_true", help="skip the opt-in kernel variants measured in subprocesses")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output vector of the last timed step to DIR/y.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(path, y, rank, world):
+    """y (the vector the timed Mult returned) as path/y.npy, or path/y_rank<r>.npy for world > 1, float64. When y is larger than
+    the rank's share of DUMP_BYTES, a fixed sample of its entries is written instead (sorted indices drawn from default_rng(0));
+    the default workload's y (2.0M dofs, 16 MB) is written whole."""
+    y = np.ascontiguousarray(y, dtype=np.float64).ravel()
+    keep = DUMP_BYTES // world // y.itemsize
+    if y.size > keep:
+        y = y[np.sort(np.random.default_rng(0).choice(y.size, keep, replace=False))]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "y.npy" if world == 1 else f"y_rank{rank}.npy"), y)
 
 
 def build_problem(n, p, warp, mesh_order=1, origin=(0.0, 0.0, 0.0), size=(1.0, 1.0, 1.0), coefficient="iso"):
@@ -208,6 +231,8 @@ def run_reference(args, rank, world):
     ref = CpuReference(prob, args.cpu_sample_elems)  # default: the whole 2M-dof mesh every step
     steps = max(1, args.steps)
     med, dts = ref.median_step(steps, warmup=max(1, min(args.warmup, 3)))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ref.y, 0, 1)
     value = float(ref.dofs_per_step / med / 1e6)
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
@@ -428,6 +453,8 @@ def main():
         b.record(stream)
     barrier()
     t_wall1 = time.time()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, yd.cpu().numpy(), rank, world)
     ms = np.array([a.elapsed_time(b) for a, b in evs])
     total_ms = float(ms.sum())
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None

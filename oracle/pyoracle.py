@@ -3,9 +3,12 @@ oracle/_ref/libpalace_qf_ref.so (the reference's own QFunction headers compiled 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference leg import this."""
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -35,14 +38,16 @@ def lib():
 
 
 def use_native_build():
-    """Timed CPU baseline only (bench.py): rebuild the oracle with -march=native ON THIS HOST into
-    oracle/_native/ and switch to it, so the baseline is not handicapped by the portable ISA level of the
-    prebuilt library. Returns True when the native build is in use."""
+    """Timed CPU baseline only (bench.py): rebuild the oracle with -march=native ON THIS HOST into a temporary
+    directory (the source tree may be read-only) and switch to it, so the baseline is not handicapped by the portable
+    ISA level of the prebuilt library. Returns True when the native build is in use."""
     global _LIB
     try:
-        subprocess.check_call(["make", "-s", "-C", _HERE, "native"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL,
-                              timeout=300)
-        _LIB = C.CDLL(os.path.join(_HERE, "_native", "liboracle.so"))
+        out = tempfile.mkdtemp(prefix="b2p_oracle_native_")
+        atexit.register(shutil.rmtree, out, ignore_errors=True)
+        subprocess.check_call(["make", "-s", "-C", _HERE, "native", "NATIVE_DIR=" + out], stdout=subprocess.DEVNULL,
+                              stderr=subprocess.DEVNULL, timeout=300)
+        _LIB = C.CDLL(os.path.join(out, "liboracle.so"))
         _LIB.orc_nd_hex_ndof.restype = C.c_int
         return True
     except Exception:

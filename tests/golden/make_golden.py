@@ -170,8 +170,35 @@ def main32curl():
     print("wrote", path, os.path.getsize(path), "bytes")
 
 
+def main_direct():
+    """tests/golden/qf_direct_golden.npz: the reference's f_apply_hdivmass_33 and f_build_geom_factor_32 on the seeded inputs of
+    test_oracle_golden.test_against_compiled_reference_headers and test_bdr_cpu.test_against_compiled_reference_32_headers, so
+    that both compare the oracle with the reference's own output where oracle/_ref cannot be built."""
+    ref = O.ref()
+    assert ref is not None, "oracle/_ref not built (needs the reference checkout)"
+    G = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "qf_golden.npz"))
+    p = lambda a: a.ctypes.data_as(C.c_void_p)
+    Q = 40
+    rng = np.random.default_rng(7)
+    qdata = np.ascontiguousarray(G["qdata"][:, :Q])
+    u, c = rng.random((3, Q)), rng.random((3, Q))
+    v, w = np.empty((3, Q)), np.empty((3, Q))
+    assert ref.ref_apply_hdivmass_33(p(np.ascontiguousarray(G["ctx_pair"])), Q, p(qdata), p(u), p(c), p(v), p(w)) == 0
+    rng = np.random.default_rng(3)
+    J = np.ascontiguousarray(rng.random((6, Q)) - 0.5) + np.array([0.8, 0, 0, 0, 1.2, 0])[:, None]
+    attr, qw = np.ones(Q), 0.2 + rng.random(Q)
+    qd = np.empty((8, Q))
+    assert ref.ref_build_geom_factor_32(Q, p(attr), p(qw), p(J), p(qd)) == 0
+    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "qf_direct_golden.npz")
+    np.savez_compressed(path, hdivmass_u=u, hdivmass_c=c, hdivmass_v=v, hdivmass_w=w, geom32_J=J, geom32_attr=attr, geom32_qw=qw,
+                        geom32_qdata=qd)
+    print("wrote", path, os.path.getsize(path), "bytes")
+
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "32":
+    if len(sys.argv) > 1 and sys.argv[1] == "direct":
+        main_direct()
+    elif len(sys.argv) > 1 and sys.argv[1] == "32":
         main32()
     elif len(sys.argv) > 1 and sys.argv[1] == "31":
         main31()

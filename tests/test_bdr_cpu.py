@@ -62,18 +62,11 @@ def test_line_elements_in_3d_are_the_padded_3d_map_too():
     assert abs((ut * v).sum() - np.linalg.norm(b - a) * (Ev @ th) ** 2 * (th @ Cm @ th)) < 1e-13
 
 
-@pytest.mark.skipif(O.ref() is None, reason="oracle/_ref not built (no /root/reference on this box)")
 def test_against_compiled_reference_32_headers():
-    import ctypes as C
-
-    ref = O.ref()
-    rng = np.random.default_rng(3)
-    Q = 40
-    p = lambda a: a.ctypes.data_as(C.c_void_p)
-    J = np.ascontiguousarray(rng.random((6, Q)) - 0.5) + np.array([0.8, 0, 0, 0, 1.2, 0])[:, None]
-    attr, qw = np.ones(Q), 0.2 + rng.random(Q)
-    qd = np.empty((8, Q))
-    assert ref.ref_build_geom_factor_32(Q, p(attr), p(qw), p(J), p(qd)) == 0
+    """The compiled reference's f_build_geom_factor_32 on seeded inputs, as stored by tests/golden/make_golden.py direct."""
+    D = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "qf_direct_golden.npz"))
+    J, attr, qw, qd = D["geom32_J"], D["geom32_attr"], D["geom32_qw"], D["geom32_qdata"]
+    Q = J.shape[1]
     assert _rel(bs.geom32_qdata(attr, qw, J), qd) < 1e-13
     # |J| is the area element and A the pseudo-inverse transposed: A^T Jm = I
     for i in range(Q):

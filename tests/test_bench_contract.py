@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -44,6 +46,21 @@ def test_reference_arm_runs_on_rank_zero_only():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "1", "--n", "4"],
                        capture_output=True, text=True, timeout=120, cwd=ROOT, env=dict(os.environ, RANK="1", LOCAL_RANK="1", WORLD_SIZE="2"))
     assert r.returncode == 0 and not [ln for ln in r.stdout.splitlines() if ln.startswith("{")]
+
+
+def test_dumped_outputs_of_both_arms_agree(tmp_path):
+    """--dump-outputs: the GPU arm (dry run on the emulation build) and the reference arm write y = A x of their last timed
+    step for the same seeded x on the same mesh, and the two agree."""
+    gpu, ref = tmp_path / "gpu", tmp_path / "ref"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "emu", "bench_dryrun.py"), "--no-cpu-baseline", "--dump-outputs", str(gpu)],
+                       capture_output=True, text=True, timeout=900, env=dict(os.environ, B2P_BENCH_EXPERIMENTS="0"), cwd=ROOT)
+    assert _last_json(r.stdout + r.stderr)["steps"] == 3
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--n", "3", "--steps", "2", "--warmup", "1",
+                        "--dump-outputs", str(ref)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert _last_json(r.stdout)["steps"] == 2
+    yg, yr = np.load(gpu / "y.npy"), np.load(ref / "y.npy")
+    assert yg.dtype == yr.dtype == np.float64 and yg.shape == yr.shape and yg.size > 0
+    assert np.abs(yg - yr).max() <= 1e-12 * np.abs(yr).max()
 
 
 def test_experiment_lines_precede_the_headline_line():

@@ -396,13 +396,13 @@ def test_ksp_composer_builds_the_reference_configuration(b2p_ctx, capi_mod, hier
 
 
 def test_multi_gpu_partition_independence():
-    """Runs tools/dist_check.py under torchrun on 2 GPUs when the box has them (gpurun --gpus 2)."""
+    """Runs tools/dist_check.py under torchrun on 2 GPUs when the machine has them."""
     import os
     import subprocess
     import sys
 
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs >= 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs >= 2 GPUs")
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2", "--master-addr",
                           "127.0.0.1", "--master-port", "29611", os.path.join(root, "tools", "dist_check.py")],

@@ -1,21 +1,20 @@
 """END-TO-END pin of the TETRAHEDRAL geometry / space path against numbers produced by the reference itself: the
-capacitance matrix of the two-spheres electrostatics example (/root/reference/examples/spheres/spheres.json: 14,362
+capacitance matrix of the two-spheres electrostatics example (the reference's examples/spheres/spheres.json: 14,362
 curved cubic tetrahedra TET20, H1 order 3, 66,328 dofs) that Palace's regression suite stores in
-test/data/regression/ref/spheres/terminal-C.csv. The oracle-side path -- Gmsh reader (palace_b200/host/gmsh.py), order-3
+test/data/regression/ref/spheres/terminal-C.csv. The oracle-side path -- the example mesh as palace_b200/host/gmsh.py reads it, order-3
 tet geometry q-data and the H1 tet space of palace_b200/host/tetspace.py, the reference QFunction arithmetic of the oracle,
 a Jacobi-preconditioned CG solve to 1e-13 -- reproduces all four entries to 1.4e-10 relative when the forms are integrated with the rule
 the reference uses (q_order = 2 p = 6 -> the 24-point symmetric rule, tetspace.tet_quadrature_symmetric6); with the 64-point conical
 rule of the same degree the entries sit 4e-8 ... 7e-8 away: on curved elements the integrand is not a polynomial, and the choice of
-rule is what round 1's looser pin was seeing. The remaining 1.3e-10 is uniform over the four entries (the physical constants' digits). The mesh is read from the reference tree (3.4 MB, not copied
-into this repository), so the test runs only where /root/reference exists.
+rule is what round 1's looser pin was seeing. The remaining 1.3e-10 is uniform over the four entries (the physical constants' digits). The example's
+mesh (3.4 MB as a .msh file) is stored compactly in tests/golden/spheres_mesh.npz (generator and loader:
+tests/golden/make_spheres_fixture.py): corners, connectivity and the curved lattice nodes; the straight ones are rebuilt.
 
 The same run's error-indicators.csv pins the GRAD-FLUX estimator on these curved tetrahedra (GradFluxErrorEstimator,
-/root/reference/palace/linalg/errorestimator.cpp:272-398 and drivers/electrostaticsolver.cpp:77-86): E = -grad V in ND_3 by the element-local
+palace/linalg/errorestimator.cpp:272-398 and drivers/electrostaticsolver.cpp:77-86): E = -grad V in ND_3 by the element-local
 discrete gradient, D = eps E projected onto RT_2 (mass CG to 1e-12), eta_K^2 = int_K |D - E|^2 scaled by 0.5 / E_elec per terminal,
 e_K = sqrt(mean over the two terminals). Global norm 2.9e-8 and mean 4.8e-8 relative to the stored values, minimum 6.1e-5 and maximum 1.2e-5
 (single elements; the reference's projection stops at 1e-6)."""
-import os
-
 import numpy as np
 import pytest
 import scipy.sparse as sp
@@ -25,10 +24,9 @@ from oracle import estimator as E
 
 from oracle import pyoracle as O
 from palace_b200.host import coeff as cf
-from palace_b200.host import gmsh
 from palace_b200.host import tetspace as ts
+from tests.golden import make_spheres_fixture
 
-MESH = "/root/reference/examples/spheres/mesh/spheres.msh"
 RULE = ts.tet_quadrature_symmetric6
 # test/data/regression/ref/spheres/terminal-C.csv (farads)
 # test/data/regression/ref/spheres/error-indicators.csv: Norm, Minimum, Maximum, Mean
@@ -38,7 +36,7 @@ C_REF = np.array([[+1.237445610357e-12, -4.770975738888e-13], [-4.770975738888e-
 
 @pytest.fixture(scope="module")
 def spheres():
-    m = gmsh.load_tets(MESH)
+    m = make_spheres_fixture.load_fixture()
     assert m.order == 3 and m.ne == 14362
     p = 3                                                            # spheres.json "Order": 3
     mesh = ts.TetMesh(m.verts, m.elems, m.attr)
@@ -84,7 +82,6 @@ def spheres():
     return dict(m=m, mesh=mesh, nd=nd, h1=h1, p=p, qpts=qpts, qd=qd, K=K, V=V)
 
 
-@pytest.mark.skipif(not os.path.exists(MESH), reason="needs the reference's example mesh")
 def test_capacitance_matrix_of_the_spheres_example(spheres):
     K, V = spheres["K"], spheres["V"]
     mu0, c0, L0 = 1.25663706127e-6, 299792458.0, 1.0e-2              # palace/utils/constants.hpp:22-30, "L0": 1e-2
@@ -94,7 +91,6 @@ def test_capacitance_matrix_of_the_spheres_example(spheres):
     assert rel.max() < 1e-9
 
 
-@pytest.mark.skipif(not os.path.exists(MESH), reason="needs the reference's example mesh")
 def test_error_indicators_of_the_spheres_example(spheres):
     """Vectorised over the 14,362 elements (the oracle's per-point loops, oracle/estimator.py, are held to it on a handful of them)."""
     m, mesh, nd, h1, p, qpts, qd, K = (spheres[k] for k in ("m", "mesh", "nd", "h1", "p", "qpts", "qd", "K"))
@@ -144,7 +140,6 @@ def test_error_indicators_of_the_spheres_example(spheres):
     assert abs(rel[0]) < 1e-6 and abs(rel[3]) < 1e-6 and abs(rel[1]) < 5e-4 and abs(rel[2]) < 1e-4
 
 
-@pytest.mark.skipif(not os.path.exists(MESH), reason="needs the reference's example mesh")
 def test_probe_field_of_the_spheres_example(spheres):
     """probe-E.csv: E = -grad V at (-1.49, 0, 0) cm, "just above the surface of the smaller sphere", for both terminals. The point is
     located in its curved cubic tetrahedron by Newton's method on the order-3 geometry map, E = -J^-T grad_ref V there; volts per metre
@@ -177,7 +172,6 @@ def test_probe_field_of_the_spheres_example(spheres):
         assert abs(Ev[0] / ref[k, 0] - 1) < 5e-7 and np.linalg.norm(Ev - ref[k]) < 2e-6 * np.linalg.norm(ref[k])
 
 
-@pytest.mark.skipif(not os.path.exists(MESH), reason="needs the reference's example mesh")
 def test_surface_charges_of_the_spheres_example(spheres):
     """surface-F.csv: the electric flux through each sphere for each terminal's field, Q = int eps E . n dS with n pointing into the
     domain, integrated on the CURVED boundary triangles -- each as a face of its parent cubic tetrahedron: points on the reference
